@@ -128,6 +128,19 @@ def identity_lut(p: int = 16, N: int = 2048, delta: int = 1 << 59) -> np.ndarray
     return algorithms.generate_programmable_bootstrap_glwe_lut(N, 2, p, delta, lambda x: x)
 
 
+DUMP_ROWS = 1024  # x 2049 words in float64 = 16.8 MB per dump; the whole 4096-row batch would be 67 MB
+
+
+def dump_outputs(directory: str, cts: np.ndarray) -> None:
+    """Write the output LWE ciphertexts of the last timed step to
+    `directory`/pbs_output.npy: a fixed sample of DUMP_ROWS rows (seed 0, kept
+    in ascending order), every word as a signed torus value int64(word) / 2^64
+    in float64, so that two builds can be compared output for output."""
+    rows = np.sort(np.random.default_rng(0).choice(len(cts), size=min(DUMP_ROWS, len(cts)), replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "pbs_output.npy"), cts[rows].view(np.int64).astype(np.float64) / 2.0 ** 64)
+
+
 def run_reference(args):
     """Reference arm: the reference's CPU algorithm (oracle port; the Rust
     crate cannot be built here) on all host cores, bounded sample per step."""
@@ -164,6 +177,8 @@ def run_reference(args):
         out = O.pbs_batch(keys, lut, cts, threads=cores)
     dt = time.perf_counter() - t0
     ok = bool(np.array_equal(O.decode(O.lwe_decrypt_batch(keys.glwe_sk, out), P.delta, 16), msgs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     value = sample * args.steps / dt
     desc = (f"{sample} PBS per step (of the {args.batch}-batch workload), FFT-mode oracle port (restatement of "
             f"tfhe-rs fft64 PBS, not tfhe-rs itself), {cores} threads (affinity / cgroup count, OMP_NUM_THREADS ignored)")
@@ -282,6 +297,9 @@ def run_b200(args):
     sync_all()
     wall_ms = (time.perf_counter() - wall0) * 1e3
     gpu_launches = L.b200_kernel_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        # read back before anything else reuses d_out (the KS+PBS extra below writes into it)
+        dump_outputs(args.dump_outputs, d_out.to_lwe_ciphertext_list(streams))
     clock_note = "sampled during the timed steps"
     if sampler.samples_in_region() < 2:
         # a K-step region shorter than nvidia-smi's period: keep the same load
@@ -312,7 +330,7 @@ def run_b200(args):
     # all K steps are inside the timed region, one host sync at the end. -------
     import ctypes as C
 
-    e2e_steps = max(2, args.steps)
+    e2e_steps = args.steps
     in_bytes, out_bytes = batch * (n + 1) * 8, batch * (k * N + 1) * 8
     sets = []
     for _ in range(2):
@@ -743,7 +761,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the keyswitch / KS+PBS side measurement")
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per launch of the PBS kernel from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the PBS outputs of the last timed step (rank 0) to DIR/pbs_output.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)
